@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- registration pairs/sec of the BUFFER-X hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2|C3|C4|C5|C1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2|C3|C4|C5|C1] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one BATCH of synthetic pairs (``--pairs-per-step``, default 48 C2 pairs: a
 step is ~0.28 s of GPU work, the default 20 steps a 5-6 s timed region through 48 distinct pairs per rank).  Every pair
@@ -221,6 +221,17 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, outs):
+    """BufferX.forward result tuples (pose, times, num_inliers, num_mutual_matches, num_inlier_ind, scales_used) of one
+    step -> out_dir/<name>.npy, one row per pair."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pose": np.stack([np.asarray(o[0], dtype=np.float64) for o in outs])}
+    for i, name in ((2, "num_inliers"), (3, "num_mutual_matches"), (4, "num_inlier_ind"), (5, "scales_used")):
+        arrays[name] = np.array([o[i] for o in outs], dtype=np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -238,7 +249,16 @@ def main():
     ap.add_argument("--cpu-pairs", type=int, default=2, help="whole pairs of the cpu_baseline leg (N=1 only)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--short", action="store_true", help="profiling runs under ncu: allow < 3 warm-up steps, skip the e2e legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned for rank 0's pairs (in pair order) "
+                         "as DIR/<name>.npy, float64: pose [B,4,4], num_inliers, num_mutual_matches, num_inlier_ind, "
+                         "scales_used [B].  Inputs and weights are seeded, so two builds can be compared output for output; "
+                         "the per-stage host times of the result tuple are measurements and are left out")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.impl == "ours" and not args.short:
         args.warmup = max(args.warmup, 3)
 
@@ -310,8 +330,8 @@ def main():
     def run_pipelined(mode, steps, timed):
         """`steps` batches of this rank's B pairs, DEPTH pairs in flight, then (when timed) the all-gather of the records --
         everything between two CUDA events.  mode 'dev': inputs resident in HBM; 'e2e': pinned host tensors through the
-        public forward_async()."""
-        recs, handles = [], []
+        public forward_async().  -> (ms, gathered records, result tuples of the last step in pair order)."""
+        recs, handles, last = [], [], []
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize()
         a.record()
@@ -321,6 +341,8 @@ def main():
 
         def collect(h, s, j):
             out = h.result()
+            if s == steps - 1:
+                last.append(out)
             if timed:
                 gt = host[j][2]["relt_pose"]
                 rte, rre = compute_rte(out[0], gt), compute_rre(out[0], gt)
@@ -353,7 +375,7 @@ def main():
             allrec = gather_records(np.stack(recs), steps * total_pairs, device=dev)   # the one collective of the path
         b.record()
         b.synchronize()
-        return a.elapsed_time(b), allrec
+        return a.elapsed_time(b), allrec, last
 
     ransac_stats = []
 
@@ -412,7 +434,7 @@ def main():
     if not strong:
         run_pipelined("dev", args.warmup, False)
     barrier()
-    ms_dev, allrec = run_pipelined("dev", args.steps, True)
+    ms_dev, allrec, last_outs = run_pipelined("dev", args.steps, True)
     barrier()
     # ---- timed region 2: host buffers through the public API --------------------------------------
     if args.short:
@@ -420,7 +442,7 @@ def main():
     else:
         run_pipelined("e2e", 1, False)
         barrier()
-        ms_e2e, _ = run_pipelined("e2e", args.steps, True)
+        ms_e2e, _, _ = run_pipelined("e2e", args.steps, True)
         barrier()
     sampler.stop_flag = True
 
@@ -492,6 +514,8 @@ def main():
                                               f"(measured sweep of a reduced pair, seconds per thread count: {sweep})",
                                     "stage_seconds_per_pair": {k: round(v, 4) for k, v in stages.items()},
                                     "wall_s": round(time.perf_counter() - t0, 2)}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_outs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

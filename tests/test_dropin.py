@@ -10,6 +10,7 @@ the collate-shaped dict of CPU tensors (dataset/dataloader.py:108-122), NumPy's 
 ``torch.cuda.empty_cache()`` between pairs, a new (Ns, Nt) for every pair -- against the oracle, eager and in graph mode
 (12 shapes > the 8 cached graph shapes, so the LRU eviction runs).
 """
+import json
 import os
 import subprocess
 import sys
@@ -63,16 +64,22 @@ def test_documented_pythonpath_resolves_reference_and_mirror_modules(tmp_path):
         assert res[n] is not None and res[n].startswith(ours), f"{n} must resolve to the B200 mirror, got {res[n]}"
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/utils"), reason="needs the reference checkout (build container only)")
-def test_real_reference_checkout_utils_are_not_shadowed():
+def test_real_reference_checkout_utils_are_not_shadowed(tmp_path):
+    """The same resolution in a tree with every Python file of the real reference checkout, by name
+    (tests/golden/reference_layout.json, written by tests/tools/gen_reference_golden.py), none of its code."""
+    ref = tmp_path / "BUFFER-X"
+    for rel in json.load(open(os.path.join(ROOT, "tests", "golden", "reference_layout.json"))):
+        (ref / rel).parent.mkdir(parents=True, exist_ok=True)
+        (ref / rel).write_text(f"ORIGIN = 'reference:{rel}'\n")
     code = ("import importlib.util as u, os; "
             "print([os.path.realpath(u.find_spec(n).origin) for n in ('utils.timer','utils.SE3','utils.tools','models.BUFFERX')])")
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "buffer-x_b200"), ROOT])
-    out = subprocess.run([sys.executable, "-c", code], cwd="/root/reference", env=env, capture_output=True, text=True, timeout=300)
+    out = subprocess.run([sys.executable, "-c", code], cwd=str(ref), env=env, capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr
     paths = eval(out.stdout.strip().splitlines()[-1])
-    assert all(p.startswith("/root/reference/utils/") for p in paths[:3]) and paths[3].startswith(os.path.realpath(ROOT))
+    utils = os.path.join(os.path.realpath(str(ref)), "utils") + os.sep
+    assert all(p.startswith(utils) for p in paths[:3]) and paths[3].startswith(os.path.realpath(ROOT))
 
 
 # ------------------------------------------------------------------------------------------------ GPU
